@@ -15,6 +15,10 @@ run is 2 client-rounds in 6583.64 s on an unnamed CPU (BASELINE.md).
   python -m torch.distributed.run --nproc-per-node 8 ... bench.py --gpus 8 --steps 5 --warmup 3
   python bench.py --impl reference    # the unmodified reference, if it can be installed
   python bench.py --impl baseline     # same pipeline on NCCL + cuDNN/cuBLAS (the bar to beat)
+  python bench.py --dump-outputs DIR  # also write the last timed round's results as DIR/<name>.npy
+
+Inputs are seeded (synthetic data, model init, key pair and encryption randomness), so runs with the same
+arguments see identical inputs and two builds can be compared through their --dump-outputs files.
 """
 import argparse
 import json
@@ -26,6 +30,24 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
 REF_CLIENT_ROUNDS_PER_SEC = 2.0 / 6583.64   # BASELINE.md: 1 round, 2 clients, 6583.64 s
+DUMP_MODEL_MAX = 1 << 22                     # float32 values of the global model written by --dump-outputs (16 MB)
+
+
+def round_outputs(run):
+    """What a caller of ``run_round`` receives from the last round, as float arrays: the averaged global model
+    that was decrypted and installed (a fixed, seeded sample of DUMP_MODEL_MAX values when it is larger) and the
+    round record's training loss and accuracy."""
+    import numpy as np
+    import torch
+
+    flat = run.pack.flat.detach().float()
+    if flat.numel() > DUMP_MODEL_MAX:
+        pick = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_MODEL_MAX]
+        flat = flat[pick.sort().values.to(flat.device)]
+    rec = run.history[-1]
+    return {"global_model": flat.cpu().numpy().astype(np.float32),
+            "loss": np.array([rec["loss"]], dtype=np.float64),
+            "accuracy": np.array([rec["accuracy"]], dtype=np.float64)}
 
 
 def reference_arm(args):
@@ -67,7 +89,12 @@ def main():
                     help="skip the NCCL + cuDNN arm that the ours arm also times and reports as own_baseline")
     ap.add_argument("--dtype", default="bf16", choices=["bf16", "fp8"],
                     help="fp8: e4m3 1x1 convolutions for the ResNets (BASELINE configs[4]); the headline config is bf16")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed rounds, write what the last one computed (global model, loss, accuracy) "
+                         "as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     if args.impl == "reference":
         return reference_arm(args)
 
@@ -122,9 +149,10 @@ def main():
             ms, wall = float(t[0]), float(t[1]) / 1e3
         return ms, wall
 
-    def measure(impl, steps, warmup, with_clocks):
+    def measure(impl, steps, warmup, with_clocks, with_outputs=False):
         """Both passes (end to end, then device-only) of one implementation: "ours" (tcgen05 engine + fused
-        ciphertext all-reduce) or "baseline" (the same pipeline on cuDNN/cuBLAS + NCCL all-reduce + mod kernel)."""
+        ciphertext all-reduce) or "baseline" (the same pipeline on cuDNN/cuBLAS + NCCL all-reduce + mod kernel).
+        ``with_outputs``: also return, on the host, what the last device-only round computed."""
         nn_backend = args.nn_backend
         if impl == "baseline":
             nn_backend = "cudnn"
@@ -138,7 +166,8 @@ def main():
         transport = "nccl" if impl == "baseline" else (args.transport or "fused")
         cfg = FLConfig(model=args.model, he_preset=args.he_preset, local_epochs=args.local_epochs,
                        steps_per_epoch=args.steps_per_epoch, val_steps=args.val_steps, clients=world,
-                       nn_backend=nn_backend, transport=transport, device="cuda", dtype=args.dtype)
+                       nn_backend=nn_backend, transport=transport, device="cuda", dtype=args.dtype,
+                       deterministic_crypto=True)
         if args.model.startswith("resnet"):
             cfg.image_size, cfg.num_classes = 224, 1000
         run = FederatedRunner(cfg, rank=rank, world=world, device=device)
@@ -192,9 +221,11 @@ def main():
         res["dev_ms"], res["dev_wall"] = dev_ms, dev_wall
         res["value"] = world * steps / (dev_ms / 1e3)
         res["shard_mb"] = (per - nval) * cfg.image_size * cfg.image_size * cfg.in_channels / 1e6
+        if with_outputs:
+            res["outputs"] = round_outputs(run)
         return res
 
-    m = measure(args.impl, args.steps, args.warmup, True)
+    m = measure(args.impl, args.steps, args.warmup, True, with_outputs=args.dump_outputs is not None)
     cfg, run = m["cfg"], m["run"]
     own_baseline = None
     if args.impl == "ours" and not args.no_own_baseline:
@@ -250,6 +281,12 @@ def main():
         if own_baseline is not None:
             out["own_baseline"] = own_baseline
             out["vs_own_baseline"] = value / own_baseline["value"]
+        if args.dump_outputs is not None:
+            import numpy as np
+
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            for name, arr in m["outputs"].items():
+                np.save(os.path.join(args.dump_outputs, name + ".npy"), arr)
         os.write(result_fd, (json.dumps(out) + "\n").encode())
     if world > 1:
         dist.destroy_process_group()

@@ -15,8 +15,8 @@
 //   conv_wgrad    : dW[r,s] = sum_m X[m+off,:]^T dY[m,:]. Both operands are consumed in their
 //                   native [P, C] layout as MN-major UMMA operands (pixels = K), so no transposed
 //                   copies exist; taps are stacked along M (128/C tap atoms per MMA group), split-K
-//                   over pixels, fp32 vector-RED into a [9*C+1, Co] buffer whose extra row is the
-//                   bias gradient (an all-ones tap atom).
+//                   over pixels: per-CTA partial sums, added to a [9*C+1, Co] buffer in a fixed order
+//                   (deterministic); the extra row is the bias gradient (an all-ones tap atom).
 //
 // Warp roles: epilogue warps first (TMEM -> registers -> global; 8 in the tap-GEMM kernel, 4 in wgrad),
 // then the TMA producer warp, then the MMA issuer warp (+TMEM owner). The two single-thread roles get the highest
@@ -782,8 +782,9 @@ void conv_fwd_pool_pair(const void* X, const void* Wf, const float* bias, void* 
 // of stages, so each X segment is fetched ONCE and serves filter rows r = 2, 1, 0 on three
 // consecutive steps; the tap column s is a row offset of the MMA descriptor (LBO = one pixel).
 // 3-D tensor maps (C, W, B*H) keep chunks inside an image row (out-of-range columns zero-fill).
-// Split over (image, strip, row range); fp32 vector-RED of the partial sums into a [9*C+1, Co]
-// buffer whose last row is the bias gradient (an all-ones A tile).
+// Split over (image, strip, row range). Every CTA stores its partial sums ([9*C+1, Co], the last row is the bias
+// gradient: an all-ones A tile) to its own slice of a workspace; splitk_sum_kernel then adds the slices to dW32 in
+// CTA order, so the result is the same on every run (fp32 RED of the partials rounded in arrival order).
 // ------------------------------------------------------------------------------------------
 #ifndef HEFL_WGRAD_OCC3
 #define HEFL_WGRAD_OCC3 0     // 1: allow three wgrad CTAs per SM (validated build flag, see WgradCfg::OCC)
@@ -797,7 +798,7 @@ struct WgradArgs {
   int units;        // B * strips * rsplit
   int nchunks;      // FLAT: ceil(B*H*W / 64)
   int Co;           // total output channels (row pitch of dW32)
-  float* dW32;      // [9*CK + 1][Co] fp32, accumulated with vector RED
+  float* part;      // [gridDim.x][9*CK + 1][Co] fp32: one partial sum per CTA
 };
 
 // FLAT = small feature maps (W <= 32): a 64-pixel chunk of one image row would be mostly padding, so
@@ -1025,12 +1026,10 @@ wgrad_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CU
           float v[32];
           tmem_ld32(tmem_base + lane_base + acc * COT + ch * 32, v);
           if (valid) {
-            float* dst = a.dW32 + (size_t)R * a.Co + co0 + ch * 32;
+            float* dst = a.part + ((size_t)blockIdx.x * (9 * CK + 1) + R) * a.Co + co0 + ch * 32;
 #pragma unroll
             for (int c = 0; c < 32; c += 4)
-              asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + c), "f"(v[c]), "f"(v[c + 1]),
-                           "f"(v[c + 2]), "f"(v[c + 3])
-                           : "memory");
+              *reinterpret_cast<float4*>(dst + c) = make_float4(v[c], v[c + 1], v[c + 2], v[c + 3]);
           }
         }
       }
@@ -1078,55 +1077,116 @@ static CUtensorMap make_map_3d_strided(const void* ptr, uint64_t C, uint64_t W, 
   return m;
 }
 
+// dst[i] += part[0][i] + part[1][i] + ... + part[splits-1][i], summed in that order whatever the launch timing
+// (32 x kSumRows threads per 32 elements: each thread sums every kSumRows-th partial, so at most a few dependent L2
+// round trips per thread; the kSumRows column sums are then added in row order)
+constexpr int kSumRows = 16;
+__global__ void __launch_bounds__(32 * kSumRows) splitk_sum_kernel(const float* __restrict__ part, int splits, int n,
+                                                                   float* __restrict__ dst) {
+  __shared__ float col[kSumRows][32];
+  pdl_prologue();
+  const int i = blockIdx.x * 32 + threadIdx.x;
+  float acc = 0.f;
+  if (i < n)
+#pragma unroll 8
+    for (int s = threadIdx.y; s < splits; s += kSumRows) acc += part[(size_t)s * n + i];
+  col[threadIdx.y][threadIdx.x] = acc;
+  __syncthreads();
+  if (threadIdx.y == 0 && i < n) {
+    float v = col[0][threadIdx.x];
+#pragma unroll
+    for (int y = 1; y < kSumRows; ++y) v += col[y][threadIdx.x];
+    dst[i] += v;
+  }
+}
+
 template <int CK, int COT, bool FLAT>
-static void launch_wgrad(const __nv_bfloat16* X, const __nv_bfloat16* DY, int B, int H, int W, int Co, float* dW32,
-                         cudaStream_t st) {
-  using Cfg = WgradCfg<CK, COT, FLAT>;
+static WgradArgs wgrad_args(int B, int H, int W, int Co) {
   WgradArgs a{};
   a.H = H; a.W = W; a.Ho = H - 2;
   a.strips = (W - 2 + 63) / 64;
-  const int cot = Co / COT;
   // units of <= 16 image rows, dealt round-robin: load imbalance <= one unit, ring warm-up 2/16
   a.rows_per = a.Ho < 16 ? a.Ho : 16;
   a.rsplit = (a.Ho + a.rows_per - 1) / a.rows_per;
   a.units = B * a.strips * a.rsplit;
-  const int P = B * H * W;
-  a.nchunks = (P + 63) / 64;
+  a.nchunks = (B * H * W + 63) / 64;
   a.Co = Co;
-  a.dW32 = dW32;
+  return a;
+}
+
+// number of CTAs along the pixel axis = number of partial sums
+template <int CK, int COT, bool FLAT>
+static int wgrad_splits(int B, int H, int W, int Co) {
+  using Cfg = WgradCfg<CK, COT, FLAT>;
+  const WgradArgs a = wgrad_args<CK, COT, FLAT>(B, H, W, Co);
+  const int total_steps = FLAT ? a.nchunks : a.units * (a.rows_per + 2);
+  // every CTA pays a fixed epilogue (the store of all accumulators): give each at least a few steps
+  int gx = total_steps / (FLAT ? 6 : 24);
+  if (gx > num_sms() * Cfg::OCC / (Co / COT)) gx = num_sms() * Cfg::OCC / (Co / COT);
+  if (gx > (FLAT ? a.nchunks : a.units)) gx = FLAT ? a.nchunks : a.units;
+  return gx < 1 ? 1 : gx;
+}
+
+template <int CK, int COT, bool FLAT>
+static void launch_wgrad(const __nv_bfloat16* X, const __nv_bfloat16* DY, int B, int H, int W, int Co, float* dW32,
+                         float* part, cudaStream_t st) {
+  using Cfg = WgradCfg<CK, COT, FLAT>;
+  WgradArgs a = wgrad_args<CK, COT, FLAT>(B, H, W, Co);
+  a.part = part;
+  const int P = B * H * W;
   CUtensorMap tmX, tmD;
-  int total_steps;
   if (FLAT) {
     tmX = make_map(X, CK, (uint64_t)P, (uint64_t)CK * 2, CK, Cfg::XROWS);
     tmD = make_map(DY, Co, (uint64_t)P, (uint64_t)Co * 2, COT, 64);
-    total_steps = a.nchunks;
   } else {
     tmX = Cfg::PACK4 ? make_map_3d_strided(X, 64, W, (uint64_t)B * H, 32, (uint64_t)W * 32, 64, Cfg::XROWS)
                      : make_map_3d(X, CK, W, (uint64_t)B * H, CK, Cfg::XROWS);
     tmD = make_map_3d(DY, Co, W, (uint64_t)B * H, COT, 64);
-    total_steps = a.units * (a.rows_per + 2);
   }
   auto kern = wgrad_kernel<CK, COT, FLAT>;
   cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, Cfg::SMEM);
-  // every CTA pays a fixed epilogue (fp32 RED of all accumulators): give each at least a few steps
-  int gx = total_steps / (FLAT ? 6 : 24);
-  if (gx > num_sms() * Cfg::OCC / cot) gx = num_sms() * Cfg::OCC / cot;
-  if (gx > (FLAT ? a.nchunks : a.units)) gx = FLAT ? a.nchunks : a.units;
-  if (gx < 1) gx = 1;
-  dim3 grid(gx, cot);
-  launch_pdl(kern, grid, dim3(192), Cfg::SMEM, st, tmX, tmD, a);
+  const int gx = wgrad_splits<CK, COT, FLAT>(B, H, W, Co);
+  launch_pdl(kern, dim3(gx, Co / COT), dim3(192), Cfg::SMEM, st, tmX, tmD, a);
+  hefl::cuda::note_launch();
+  const int n = (9 * CK + 1) * Co;
+  launch_pdl(splitk_sum_kernel, dim3((n + 31) / 32), dim3(32, kSumRows), 0, st, part, gx, n, dW32);
   hefl::cuda::note_launch();
 }
 
-void conv_wgrad(const void* X, const void* DY, float* dW32, int B, int H, int W, int CK, int Co, cudaStream_t st) {
+template <int CK, int COT, bool FLAT>
+struct WgradShape {
+  static constexpr int ck = CK, cot = COT;
+  static constexpr bool flat = FLAT;
+};
+
+// the (CK, Co) -> kernel instance table, shared by the launcher and the workspace query
+template <class F>
+static auto wgrad_dispatch(int CK, int Co, int W, F&& f) {
+  const bool flat = W <= 32 && CK != 16;
+  if (CK == 16 && Co == 32) return f(WgradShape<16, 32, false>{});
+  if (CK == 32 && Co == 32) return flat ? f(WgradShape<32, 32, true>{}) : f(WgradShape<32, 32, false>{});
+  if (CK == 32 && Co == 64) return flat ? f(WgradShape<32, 64, true>{}) : f(WgradShape<32, 64, false>{});
+  if (CK == 64 && (Co == 64 || Co == 128)) return flat ? f(WgradShape<64, 64, true>{}) : f(WgradShape<64, 64, false>{});
+  throw std::runtime_error("conv_wgrad: unsupported (CK, Co)");
+}
+
+size_t conv_wgrad_part_floats(int B, int H, int W, int CK, int Co) {
+  const int splits = wgrad_dispatch(CK, Co, W, [&](auto s) {
+    using S = decltype(s);
+    return wgrad_splits<S::ck, S::cot, S::flat>(B, H, W, Co);
+  });
+  return (size_t)splits * (9 * CK + 1) * Co;
+}
+
+void conv_wgrad(const void* X, const void* DY, float* dW32, float* part, int B, int H, int W, int CK, int Co,
+                cudaStream_t st) {
   const auto* x = reinterpret_cast<const __nv_bfloat16*>(X);
   const auto* d = reinterpret_cast<const __nv_bfloat16*>(DY);
-  const bool flat = W <= 32 && CK != 16;
-  if (CK == 16 && Co == 32) launch_wgrad<16, 32, false>(x, d, B, H, W, Co, dW32, st);
-  else if (CK == 32 && Co == 32) flat ? launch_wgrad<32, 32, true>(x, d, B, H, W, Co, dW32, st) : launch_wgrad<32, 32, false>(x, d, B, H, W, Co, dW32, st);
-  else if (CK == 32 && Co == 64) flat ? launch_wgrad<32, 64, true>(x, d, B, H, W, Co, dW32, st) : launch_wgrad<32, 64, false>(x, d, B, H, W, Co, dW32, st);
-  else if (CK == 64 && (Co == 64 || Co == 128)) flat ? launch_wgrad<64, 64, true>(x, d, B, H, W, Co, dW32, st) : launch_wgrad<64, 64, false>(x, d, B, H, W, Co, dW32, st);
-  else throw std::runtime_error("conv_wgrad: unsupported (CK, Co)");
+  wgrad_dispatch(CK, Co, W, [&](auto s) {
+    using S = decltype(s);
+    launch_wgrad<S::ck, S::cot, S::flat>(x, d, B, H, W, Co, dW32, part, st);
+    return 0;
+  });
 }
 
 }  // namespace nn

@@ -22,7 +22,11 @@ void conv_fwd_pool_pair(const void* X, const void* Wf, const float* bias, void* 
 void conv_set_debug(int mask);
 void conv_dgrad(const void* dY, const void* Wd, void* dX, int B, int H, int W, int CK, int CO, const uint8_t* up_amax,
                 int up_W, cudaStream_t st);
-void conv_wgrad(const void* X, const void* DY, float* dW32, int B, int H, int W, int CK, int Co, cudaStream_t st);
+// dW32 += the weight gradient. part: workspace of conv_wgrad_part_floats(...) floats for the per-CTA partial sums,
+// which are added in a fixed order, so the result does not change from run to run.
+size_t conv_wgrad_part_floats(int B, int H, int W, int CK, int Co);
+void conv_wgrad(const void* X, const void* DY, float* dW32, float* part, int B, int H, int W, int CK, int Co,
+                cudaStream_t st);
 
 // Dense head (Flatten -> Dense/ReLU -> Dense/ReLU -> Dense -> softmax-CE) forward + backward.
 void head_forward_backward(const void* feat, const float* W1, const float* b1, const float* W2, const float* b2,
@@ -40,8 +44,10 @@ void wgrad0_gather(const void* X, const void* g, const uint8_t* amax, float* dW,
                    cudaStream_t st);
 // the same gradient as four masked GEMMs on the tensor cores (wgrad0_mma.cu); needs the s-packed layer-1 input
 bool wgrad0_mma_supported(int W, int Wp, int CK, int Ci, int Co);
-void wgrad0_mma(const void* X, const void* g, const uint8_t* amax, float* dW, int B, int H, int W, int Hp, int Wp,
-                cudaStream_t st);
+// (deterministic like conv_wgrad: part holds wgrad0_mma_part_floats(B, Hp) floats of per-CTA partial sums)
+size_t wgrad0_mma_part_floats(int B, int Hp);
+void wgrad0_mma(const void* X, const void* g, const uint8_t* amax, float* dW, float* part, int B, int H, int W, int Hp,
+                int Wp, cudaStream_t st);
 // ---- general tcgen05 GEMMs for the ResNet convolutions (gemm_tcgen05.cu) ----
 // C[rows_out, N] (bf16) = sum_{t < taps} A[m + shifts[t], K] . B[t*N + n, K]^T. padded != 0: A rows index a zero-padded
 // [Bn][H+2][W+2] grid and only interior pixels are written (to the dense [Bn*H*W, N] output). fp8: A and B hold e4m3

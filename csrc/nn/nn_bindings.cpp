@@ -137,7 +137,11 @@ void conv_wgrad(const Tensor& X, const Tensor& DY, Tensor dW32, int64_t B, int64
   const int64_t P = B * H * W;
   TORCH_CHECK(X.numel() == P * CK && DY.numel() == P * Co, "X must be [B*H*W,CK] and DY [B*H*W,Co]");
   TORCH_CHECK(dW32.is_cuda() && dW32.scalar_type() == at::kFloat && dW32.numel() >= (9 * CK + 1) * Co, "dW32 too small");
-  hefl::nn::conv_wgrad(X.data_ptr(), DY.data_ptr(), dW32.data_ptr<float>(), (int)B, (int)H, (int)W, (int)CK, (int)Co, cur());
+  // per-CTA partial sums, summed in a fixed order by the launcher (from the caching allocator: graph-capture safe)
+  Tensor part = at::empty({(int64_t)hefl::nn::conv_wgrad_part_floats((int)B, (int)H, (int)W, (int)CK, (int)Co)},
+                          dW32.options());
+  hefl::nn::conv_wgrad(X.data_ptr(), DY.data_ptr(), dW32.data_ptr<float>(), part.data_ptr<float>(), (int)B, (int)H, (int)W,
+                       (int)CK, (int)Co, cur());
 }
 
 void preprocess_u8(const Tensor& x, const c10::optional<Tensor>& theta, Tensor X, int64_t aug_seed,
@@ -245,8 +249,9 @@ void wgrad0_gather(const Tensor& X, const Tensor& g, const Tensor& amax, Tensor 
   TORCH_CHECK(X.numel() >= B * H * W * 16 && g.numel() == B * Hp * Wp * 32 && amax.numel() == g.numel(), "shape mismatch");
   TORCH_CHECK(amax.scalar_type() == at::kByte && dW32.scalar_type() == at::kFloat && dW32.numel() >= (9 * 16 + 1) * 32, "dtype / size");
   if (spack && hefl::nn::wgrad0_mma_supported((int)W, (int)Wp, 16, 3, 32)) {      // s-packed input: masked GEMMs on the tensor cores
-    hefl::nn::wgrad0_mma(X.data_ptr(), g.data_ptr(), amax.data_ptr<uint8_t>(), dW32.data_ptr<float>(), (int)B, (int)H, (int)W,
-                         (int)Hp, (int)Wp, cur());
+    Tensor part = at::empty({(int64_t)hefl::nn::wgrad0_mma_part_floats((int)B, (int)Hp)}, dW32.options());
+    hefl::nn::wgrad0_mma(X.data_ptr(), g.data_ptr(), amax.data_ptr<uint8_t>(), dW32.data_ptr<float>(), part.data_ptr<float>(),
+                         (int)B, (int)H, (int)W, (int)Hp, (int)Wp, cur());
     return;
   }
   hefl::nn::wgrad0_gather(X.data_ptr(), g.data_ptr(), amax.data_ptr<uint8_t>(), dW32.data_ptr<float>(), (int)B, (int)H,

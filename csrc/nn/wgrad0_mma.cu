@@ -24,8 +24,9 @@
 //     selector, the table is 0xFF at entry 4 + c, so one instruction yields the 16-bit masks of two channels;
 //   * 8 warps = 8 x 16 pooled pixels of a strip; each keeps the full 48 x 32 fp32 tile (48 registers). At the end
 //     every warp parks its tile in shared memory (no atomics: fp32 shared atomics are CAS loops on this part and
-//     cost 29 % of the first version), the tiles are summed, and one fp32 RED per CTA and useful element goes to
-//     the split-K buffer the other weight-gradient kernels use. The bias gradient is the sum of the active g,
+//     cost 29 % of the first version), the tiles are summed in warp order and each CTA stores its 28 x 32 partial
+//     sums; wgrad0_sum_kernel adds them, in CTA order, to the split-K buffer the other weight-gradient kernels
+//     use (same result on every run, unlike an fp32 RED per CTA). The bias gradient is the sum of the active g,
 //     taken in the mask pass.
 //
 // (Why mma.sync and not tcgen05 here: the B operand is produced by the CUDA cores, M x N is 48 x 32 and the
@@ -58,6 +59,14 @@ constexpr int kGs = kPx * 64;           // one masked tile
 constexpr int kBarOff = kRing * kSlot + 2 * kGst + 2 * kCst + 4 * kGs;
 constexpr int kSmem = kBarOff + 64;     // 104 KB -> 2 CTAs / SM
 constexpr int kPartStride = 40;         // floats per row of a parked accumulator tile (bank spread)
+constexpr int kOut = 28 * 32;           // useful gradient elements: 27 (r, q, ci) rows + the bias row, x 32 co
+
+// dW32 row of partial-sum row ``row``: tap * CK + ci for the 27 weight rows, 9 * CK for the bias
+__device__ __forceinline__ int wgrad0_out_row(int row) {
+  if (row == 27) return 9 * 16;
+  const int r = row / 9, m = row - r * 9, q = m / 3, ci = m - q * 3;
+  return (r * 3 + q) * 16 + ci;
+}
 constexpr int kPart = 48 * kPartStride + 32;   // one warp's tile + its bias sums
 static_assert(8 * kPart * 4 <= kBarOff, "parked tiles must fit in the operand buffers");
 
@@ -77,7 +86,7 @@ __device__ __forceinline__ void mma16816(float (&d)[4], const uint32_t (&a)[4], 
 
 __global__ void __launch_bounds__(kT, 2)
 wgrad0_mma_kernel(const __grid_constant__ CUtensorMap tmX, const __nv_bfloat16* __restrict__ g,
-                  const uint8_t* __restrict__ amax, float* __restrict__ dW, int B, int H, int W, int Hp, int Wp) {
+                  const uint8_t* __restrict__ amax, float* __restrict__ part, int B, int H, int W, int Hp, int Wp) {
   extern __shared__ __align__(1024) uint8_t sm[];
   uint8_t* ring = sm;
   uint8_t* gst = ring + kRing * kSlot;
@@ -217,9 +226,9 @@ wgrad0_mma_kernel(const __grid_constant__ CUtensorMap tmX, const __nv_bfloat16* 
   }
 
   // every warp parks its tile (all copies have landed: the last strip requests nothing), then a plain sum
-  float* part = reinterpret_cast<float*>(sm);
+  float* tiles = reinterpret_cast<float*>(sm);
   {
-    float* mine = part + warp * kPart;
+    float* mine = tiles + warp * kPart;
     const int gq = lane >> 2, tq = lane & 3;
 #pragma unroll
     for (int r = 0; r < 3; ++r)
@@ -239,21 +248,40 @@ wgrad0_mma_kernel(const __grid_constant__ CUtensorMap tmX, const __nv_bfloat16* 
     }
   }
   __syncthreads();
-  for (int idx = tid; idx < 28 * 32; idx += kT) {
+  for (int idx = tid; idx < kOut; idx += kT) {
     const int row = idx >> 5, co = idx & 31;
-    int src, out_row;
+    int src;
     if (row < 27) {
-      const int r = row / 9, m = row - r * 9, q = m / 3, ci = m - q * 3;
+      const int r = row / 9, m = row - r * 9;
       src = (r * 16 + m) * kPartStride + co;
-      out_row = (r * 3 + q) * 16 + ci;                       // dW32 rows: tap * CK + ci
     } else {
-      src = 48 * kPartStride + co;
-      out_row = 9 * 16;                                      // bias row
+      src = 48 * kPartStride + co;                           // bias sums
     }
     float v = 0.f;
 #pragma unroll
-    for (int w = 0; w < 8; ++w) v += part[w * kPart + src];
-    atomicAdd(&dW[out_row * 32 + co], v);
+    for (int w = 0; w < 8; ++w) v += tiles[w * kPart + src];
+    part[(size_t)blockIdx.x * kOut + idx] = v;
+  }
+}
+
+// dW[wgrad0_out_row(row)][co] += sum of the CTAs' partial sums, in CTA order (one block per row)
+// (32 x kSumRows threads per row: few dependent L2 round trips per thread, on the tail of the training step)
+constexpr int kSumRows = 32;
+__global__ void __launch_bounds__(32 * kSumRows) wgrad0_sum_kernel(const float* __restrict__ part, int splits,
+                                                                   float* __restrict__ dW) {
+  __shared__ float col[kSumRows][32];
+  pdl_prologue();
+  const int idx = blockIdx.x * 32 + threadIdx.x;
+  float acc = 0.f;
+#pragma unroll 8
+  for (int s = threadIdx.y; s < splits; s += kSumRows) acc += part[(size_t)s * kOut + idx];
+  col[threadIdx.y][threadIdx.x] = acc;
+  __syncthreads();
+  if (threadIdx.y == 0) {
+    float v = col[0][threadIdx.x];
+#pragma unroll
+    for (int y = 1; y < kSumRows; ++y) v += col[y][threadIdx.x];
+    dW[wgrad0_out_row(blockIdx.x) * 32 + threadIdx.x] += v;
   }
 }
 
@@ -290,21 +318,32 @@ bool wgrad0_mma_supported(int W, int Wp, int CK, int Ci, int Co) {
   return on && CK == 16 && Ci <= 3 && Co == 32 && W <= 256 && (W & 1) == 0 && Wp <= kPx && Wp >= 1;
 }
 
-void wgrad0_mma(const void* X, const void* g, const uint8_t* amax, float* dW, int B, int H, int W, int Hp, int Wp,
-                cudaStream_t st) {
+static int wgrad0_mma_grid(int B, int Hp) {
   static int sms = 0;
   if (!sms) {
     int dev = 0;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  }
+  return sms * 2 < B * Hp ? sms * 2 : B * Hp;
+}
+
+size_t wgrad0_mma_part_floats(int B, int Hp) { return (size_t)wgrad0_mma_grid(B, Hp) * kOut; }
+
+void wgrad0_mma(const void* X, const void* g, const uint8_t* amax, float* dW, float* part, int B, int H, int W, int Hp,
+                int Wp, cudaStream_t st) {
+  static bool attrs = false;
+  if (!attrs) {
     cudaFuncSetAttribute(wgrad0_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmem);
     cudaFuncSetAttribute(wgrad0_mma_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, 100);
+    attrs = true;
   }
   const CUtensorMap tmX = make_row_map(X, (uint64_t)B * H * (W / 2), (uint32_t)(W / 2));
-  int grid = sms * 2;
-  if (grid > B * Hp) grid = B * Hp;
-  launch_pdl(wgrad0_mma_kernel, dim3(grid), dim3(kT), kSmem, st, tmX, reinterpret_cast<const __nv_bfloat16*>(g), amax, dW,
-             B, H, W, Hp, Wp);
+  const int grid = wgrad0_mma_grid(B, Hp);
+  launch_pdl(wgrad0_mma_kernel, dim3(grid), dim3(kT), kSmem, st, tmX, reinterpret_cast<const __nv_bfloat16*>(g), amax,
+             part, B, H, W, Hp, Wp);
+  hefl::cuda::note_launch();
+  launch_pdl(wgrad0_sum_kernel, dim3(kOut / 32), dim3(32, kSumRows), 0, st, part, grid, dW);
   hefl::cuda::note_launch();
 }
 

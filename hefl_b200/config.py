@@ -61,7 +61,8 @@ class FLConfig:
                                               # get_sk only in decrypt (:284). -1: rank 0 generates and hands sk to every
                                               # rank (every client can decrypt; weaker, kept for experiments)
     deterministic_crypto: bool = False        # tests / debugging ONLY: derive the key pair and every encryption seed from
-                                              # ``seed`` (public!) instead of OS entropy, so runs are bit-reproducible
+                                              # ``seed`` (public!) instead of OS entropy, so runs are bit-reproducible;
+                                              # bench.py sets it (synthetic data, reproducible inputs), never for real data
     pairwise_masks: bool = False              # add PRG masks (X25519-agreed pair seeds, +/- per pair) to each client's
                                               # ciphertext before the all-reduce; they cancel in the sum
     allow_dropouts: bool = False              # clients may sit a round out (participation mask): K becomes a runtime

@@ -12,7 +12,7 @@ Replaces Keras' ``model.fit`` compute path (FLPyfhelin.py:118-136, :193) for the
             head_forward_backward (Dense 128-64-C + softmax CE, forward AND backward, one launch on a
                                    cluster of 8 CTAs)
   backward  unpool_relu / conv_dgrad chain on the main stream (layers 6..2),
-            conv_wgrad (tcgen05, MN-major operands, split-K RED) on a side stream,
+            conv_wgrad (tcgen05, MN-major operands, split-K partials summed in a fixed order) on a side stream,
             layer 1: wgrad0_gather straight from the pooled gradient (no un-pool, no dY tensor): four
                      masked GEMMs on the tensor cores (wgrad0_mma.cu), FP32-pipe gather as the fallback
   update    conv_grad_finalize + Adam + conv_weight_relayout: layers 2..6 and the head on the side

@@ -32,6 +32,11 @@ def test_own_arm_prints_exactly_one_json_line_without_cuda():
     assert len(lines) == 1 and "error" in json.loads(lines[0])
 
 
+def test_steps_below_one_are_refused():
+    r = _run("--steps", "0")
+    assert r.returncode == 2 and not r.stdout.strip() and "--steps" in r.stderr
+
+
 def test_graft_entry_exposes_build_and_smoke():
     sys.path.insert(0, ROOT)
     import __graft_entry__ as g

@@ -85,7 +85,10 @@ def test_conv_wgrad_matches_torch(B, H, Ci, CK, Co):
     P = B * H * H
     dW32 = torch.zeros((9 * CK + 1) * Co, dtype=torch.float32, device="cuda")
     ops.conv_wgrad(x.view(-1, CK), dY.view(-1, Co), dW32, B, H, H, CK, Co)
+    again = torch.zeros_like(dW32)
+    ops.conv_wgrad(x.view(-1, CK), dY.view(-1, Co), again, B, H, H, CK, Co)
     torch.cuda.synchronize()
+    assert torch.equal(dW32, again)                  # split-K partials are summed in a fixed order
     xr = x[..., :Ci].float().permute(0, 3, 1, 2).requires_grad_(False)
     wref = torch.nn.grad.conv2d_weight(xr, (Co, Ci, 3, 3), dyv.float())
     got = dW32[: 9 * CK * Co].view(9, CK, Co)[:, :Ci, :].permute(2, 1, 0).reshape(Co, Ci, 3, 3)
@@ -342,7 +345,10 @@ def test_wgrad0_masked_gemm_matches_gather_and_autograd(B, H):
     d_gat = torch.zeros_like(d_mma)
     ops.wgrad0_gather(X, gflat, amax, d_mma.view(-1), B, H, H, True)
     ops.wgrad0_gather(X, gflat, amax, d_gat.view(-1), B, H, H, False)
+    again = torch.zeros_like(d_mma)
+    ops.wgrad0_gather(X, gflat, amax, again.view(-1), B, H, H, True)
     torch.cuda.synchronize()
+    assert torch.equal(d_mma, again)                 # per-CTA partials are summed in a fixed order
     # same products, fp32 accumulation in a different order
     scale = d_gat.abs().max()
     assert (d_mma - d_gat).abs().max() <= 2e-5 * scale + 1e-5
